@@ -480,6 +480,21 @@ def bench_mhs(ctx, gpu, torch, dev):
     return out
 
 
+DUMP_MAX_VALUES = 1 << 23  # float32 values per dumped array: the two arrays stay under 64 MB at any GPU count
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: DIR/<name>.npy in float32 (statuses and bits are small integers, exact in float32).  An array longer
+    than DUMP_MAX_VALUES keeps only the values at DUMP_MAX_VALUES positions drawn with seed 0, in increasing order: the
+    same positions for every run of the same size."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size > DUMP_MAX_VALUES:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_VALUES, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32))
+
+
 def run_gpu(args, rank, world, local_rank):
     import numpy as np
     import torch
@@ -600,6 +615,13 @@ def run_gpu(args, rank, world, local_rank):
     dt = _max_over_ranks(dt_local, dev, world)
     value = n_global * args.steps / dt
     step_max = _max_over_ranks(per_step[-1], dev, world)
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        # what the caller of the timed path received from its last step: the gathered accept bitmap (one bit per proof of the
+        # whole batch, without the padding of each rank's words) and this rank's per-proof statuses
+        bits = np.unpackbits(g_bitmaps[(args.steps - 1) & 1].cpu().numpy().view(np.uint8), bitorder="little")
+        outputs = {"accept_bits": np.concatenate([bits[r * per_words * 64:r * per_words * 64 + n] for r in range(world)]),
+                   "status": d_status.cpu().numpy()}
 
     # ---- end to end through the host-pointer ABI ----
     h_nodes = torch.empty(n_bytes + 64, dtype=torch.uint8, pin_memory=True)
@@ -700,6 +722,8 @@ def run_gpu(args, rank, world, local_rank):
         line.update(extras)
         if world == 1 and not args.no_cpu:
             line["cpu_baseline"] = cpu_arm(131072, target_cpu_seconds=20.0, threads=host_threads())
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
         if not (status_ok and bitmap_ok and e2e_ok):
             sys.exit("verdicts differ from the expected pattern")
@@ -717,7 +741,11 @@ def main():
     ap.add_argument("--impl", default="phant_b200", choices=["phant_b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--skip-extras", action="store_true", help="only the contract workload (C2): no c3 / c4 / c5 / MH-by-size keys")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (accept_bits: the "
+                    "gathered bitmap, one value per proof; status: rank 0's per-proof statuses) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl phant_b200)")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -199,6 +199,37 @@ def py_mptize(keccak, kv):
     return keccak(node if node else b"\x80")
 
 
+# ---- inputs whose answers were computed by the reference's own compiled code (tests/golden/compiled_reference_kat.json,
+# written by tests/golden/make_compiled_reference_kat.py): changing them invalidates the stored answers
+def compiled_reference_keccak_messages():
+    """random messages of lengths 0..299 and around the 136-byte rate boundaries, up to 1200 bytes"""
+    import numpy as np
+    rng = np.random.default_rng(1)
+    return [rng.integers(0, 256, n, dtype=np.uint8).tobytes()
+            for n in list(range(0, 300)) + [407, 408, 409, 543, 544, 545, 1087, 1088, 1089, 1200]]
+
+
+def compiled_reference_secure_tries():
+    """random secure tries: sorted 32-byte keys, 33..119-byte values, 1..1000 entries -> [[(key, value)]]"""
+    import numpy as np
+    rng = np.random.default_rng(7)
+    tries = []
+    for n in (1, 2, 3, 17, 100, 1000):
+        keys = sorted(rng.integers(0, 256, 32, dtype=np.uint8).tobytes() for _ in range(n))
+        vals = [rng.integers(0, 256, int(rng.integers(33, 120)), dtype=np.uint8).tobytes() for _ in range(n)]
+        tries.append(list(zip(keys, vals)))
+    return tries
+
+
+def inputs_sha256(chunks):
+    """sha256 over length-prefixed byte strings: pins the inputs that stored answers belong to"""
+    import hashlib
+    h = hashlib.sha256()
+    for c in chunks:
+        h.update(len(c).to_bytes(8, "little") + c)
+    return h.hexdigest()
+
+
 # ---- a stand-in for phant_b200.gpu.Context that computes with the CPU oracle: lets the HOST logic above the C ABI
 # (flattening, decoding, ownership, error mapping) run in the CPU test suite; the -m gpu tests run the same host code on the device
 class OracleBackedCtx:

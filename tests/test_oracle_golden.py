@@ -3,13 +3,10 @@
 CPU-only.  If these fail nothing else in the suite means anything: the GPU parity tests compare against
 this oracle.
 """
-import os
-
 import numpy as np
 import pytest
 
-import oracle_lib
-from helpers import index_trie_items
+from helpers import compiled_reference_keccak_messages, compiled_reference_secure_tries, index_trie_items, inputs_sha256
 
 
 def test_keccak_reference_table(oracle, golden):
@@ -41,13 +38,15 @@ def test_keccak_constants(oracle):
     assert oracle.keccak256(b"\xc0").hex() == "1dcc4de8dec75d7aab85b567b6ccd41ad312451b948a7413f0a142fd40d49347"
 
 
-@pytest.mark.skipif(not os.path.exists(oracle_lib.REF_KECCAK_PATH), reason="oracle/_ref not built (no reference checkout)")
-def test_port_equals_compiled_reference_keccak(oracle):
-    """The port vs the reference's keccak.c compiled unchanged (oracle/_ref), random lengths 0..1200."""
-    rng = np.random.default_rng(1)
-    for n in list(range(0, 300)) + [407, 408, 409, 543, 544, 545, 1087, 1088, 1089, 1200]:
-        m = rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-        assert oracle.keccak256(m) == oracle.ref_keccak256(m), n
+def test_port_equals_compiled_reference_keccak(oracle, golden):
+    """The port vs the reference's keccak.c compiled unchanged (oracle/_ref; digests stored by
+    tests/golden/make_compiled_reference_kat.py), random lengths 0..1200."""
+    g = golden("compiled_reference_kat.json")
+    msgs = compiled_reference_keccak_messages()
+    assert inputs_sha256(msgs) == g["keccak_inputs_sha256"], "the messages differ from those the digests were computed for"
+    assert [len(m) for m in msgs] == [c["len"] for c in g["keccak"]]
+    for m, c in zip(msgs, g["keccak"]):
+        assert oracle.keccak256(m).hex() == c["keccak256"], len(m)
 
 
 def test_mptize_reference_roots(oracle, golden):
@@ -106,22 +105,16 @@ def test_fixture_list_roots(oracle, golden):
     assert n == 87
 
 
-@pytest.mark.skipif(not os.path.exists(oracle_lib.REF_EVMONE_PATH), reason="oracle/_ref not built (no reference checkout)")
-def test_secure_trie_equals_compiled_evmone(oracle):
-    """Random secure tries: mptize restatement vs the reference's vendored evmone MPT compiled unchanged."""
-    import ctypes as C
-    ref = C.CDLL(oracle_lib.REF_EVMONE_PATH)
-    rng = np.random.default_rng(7)
-    for n in (1, 2, 3, 17, 100, 1000):
-        keys = sorted(rng.integers(0, 256, 32, dtype=np.uint8).tobytes() for _ in range(n))
-        vals = [rng.integers(0, 256, int(rng.integers(33, 120)), dtype=np.uint8).tobytes() for _ in range(n)]
-        k, koff = oracle_lib.csr(keys, np.uint32)
-        v, voff = oracle_lib.csr(vals, np.uint64)
-        out = np.zeros(32, np.uint8)
-        ref.ref_evmone_mpt_root(k.ctypes.data_as(oracle_lib.u8p), koff.ctypes.data_as(oracle_lib.u32p),
-                                v.ctypes.data_as(oracle_lib.u8p), voff.ctypes.data_as(oracle_lib.u64p), C.c_uint64(n),
-                                out.ctypes.data_as(oracle_lib.u8p))
-        assert oracle.mptize(list(zip(keys, vals))) == out.tobytes(), n
+def test_secure_trie_equals_compiled_evmone(oracle, golden):
+    """Random secure tries: mptize restatement vs the reference's vendored evmone MPT compiled unchanged (oracle/_ref;
+    roots stored by tests/golden/make_compiled_reference_kat.py)."""
+    g = golden("compiled_reference_kat.json")
+    tries = compiled_reference_secure_tries()
+    assert inputs_sha256([k + v for kv in tries for k, v in kv]) == g["secure_trie_inputs_sha256"], \
+        "the tries differ from those the roots were computed for"
+    assert [len(kv) for kv in tries] == [c["n"] for c in g["secure_trie"]]
+    for kv, c in zip(tries, g["secure_trie"]):
+        assert oracle.mptize(kv).hex() == c["root"], len(kv)
 
 
 def test_logs_bloom_reference_vector(oracle, golden):
