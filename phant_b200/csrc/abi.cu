@@ -214,7 +214,7 @@ int phant_gpu_ctx::hash_csr(const uint8_t* d_msgs, const uint64_t* d_off, uint64
     if (int rc = d_perms.reserve(ctx, 64)) return rc;
     if (!perms_init) { CU(cudaMemsetAsync(d_perms.ptr, 0, 64, stream)); perms_init = true; } // [0] permutations, [1] block ticket
     if (int rc = d_idx.reserve(ctx, keccak_regroup_scratch_bytes(device, n))) return rc;
-    CU(launch_keccak_classify(stream, device, d_off, n, (uint32_t*)d_idx.ptr, (uint32_t*)((unsigned long long*)d_perms.ptr + 1),
+    CU(launch_keccak_classify(stream, device, d_off, nullptr, n, (uint32_t*)d_idx.ptr, (uint32_t*)((unsigned long long*)d_perms.ptr + 1),
                               (unsigned long long*)d_perms.ptr));
     stats.launches++;
     perms_pending = true;
@@ -222,7 +222,7 @@ int phant_gpu_ctx::hash_csr(const uint8_t* d_msgs, const uint64_t* d_off, uint64
     const bool regroup = !(flags & PHANT_GPU_FLAG_NO_BINNING) && variant != KECCAK_WARP && n >= 4096;
     if (regroup) {
         if (int rc = d_order.reserve(ctx, 4 * n)) return rc;
-        CU(launch_keccak_regroup(stream, device, d_off, n, (const uint32_t*)d_idx.ptr, (uint32_t*)d_order.ptr));
+        CU(launch_keccak_regroup(stream, device, d_off, nullptr, n, (const uint32_t*)d_idx.ptr, (uint32_t*)d_order.ptr));
         stats.launches++;
         order = (const uint32_t*)d_order.ptr;
     }
@@ -303,6 +303,50 @@ extern "C" int phant_gpu_keccak256_batch_async(phant_gpu_ctx* ctx, const uint8_t
 // ------------------------------------------------------------------------------------------------
 // V: proof verification
 // ------------------------------------------------------------------------------------------------
+// A CSR chain (no node_index) is verified in one pass: verify_fused.cu hashes and walks each proof in the same lane, so the
+// digests and node summaries of the two-pass path (hash_csr + walk_kernel) are never written.  Proofs are regrouped by their
+// permutation count first (keccak_kernels.cu "regrouping", per proof instead of per node), so that the 32 lanes of a warp
+// hash chains of similar length.  The two-pass path stays for deduplicated witnesses (a shared node is hashed once), for
+// the KECCAK_DIRECT / KECCAK_WARP variants and for a node buffer that is not 16-byte aligned.
+static bool fused_path(const phant_gpu_ctx* ctx, const uint8_t* nodes)
+{
+    return !(ctx->flags & (PHANT_GPU_FLAG_KECCAK_DIRECT | PHANT_GPU_FLAG_KECCAK_WARP)) && verify_fused_supported(nodes);
+}
+// `fence_and_clear`: device-pointer call -- wait for the collective still using `bitmap` (sharded calls), then zero it
+static int verify_fused(phant_gpu_ctx* ctx, const uint8_t* nodes, const uint64_t* node_off, const uint64_t* proof_first, uint64_t np,
+                        uint64_t n_nodes, uint64_t total, const uint8_t* keys32, const uint8_t* roots32, uint64_t n_roots, uint64_t* bitmap,
+                        uint8_t* status, uint64_t* val_off, uint32_t* val_len, const PeerOut* peer, bool fence_and_clear)
+{
+    if (np > 0xffffffffull) return PHANT_GPU_E_INVALID; // proof indices are 32-bit on the device
+    NvtxRange nvtx("phant:verify");
+    cudaStream_t s = ctx->stream;
+    if (int rc = ctx->d_perms.reserve(ctx, 64)) return rc;
+    if (!ctx->perms_init) { CU(cudaMemsetAsync(ctx->d_perms.ptr, 0, 64, s)); ctx->perms_init = true; } // [0] permutations, [1] block ticket
+    const uint32_t* order = nullptr;
+    if (!peer && !(ctx->flags & PHANT_GPU_FLAG_NO_BINNING) && np >= 4096) {
+        if (int rc = ctx->d_idx.reserve(ctx, keccak_regroup_scratch_bytes(ctx->device, np))) return rc;
+        if (int rc = ctx->d_order.reserve(ctx, 4 * np)) return rc;
+        CU(launch_keccak_classify(s, ctx->device, node_off, proof_first, np, (uint32_t*)ctx->d_idx.ptr,
+                                  (uint32_t*)((unsigned long long*)ctx->d_perms.ptr + 1), nullptr));
+        CU(launch_keccak_regroup(s, ctx->device, node_off, proof_first, np, (const uint32_t*)ctx->d_idx.ptr, (uint32_t*)ctx->d_order.ptr));
+        ctx->stats.launches += 2;
+        order = (const uint32_t*)ctx->d_order.ptr;
+    }
+    if (fence_and_clear) {
+        if (int rc = ctx->wait_walk_fence()) return rc; // sharded call: the previous gather of this bitmap buffer (comm.cu)
+        if (bitmap) CU(cudaMemsetAsync(bitmap, 0, ((np + 63) / 64) * 8, s));
+    }
+    ctx->time_begin(0);
+    CU(launch_verify_fused(s, ctx->device, np, nodes, node_off, proof_first, order, keys32, roots32, n_roots, bitmap, status, val_off, val_len,
+                           (unsigned long long*)ctx->d_perms.ptr, peer));
+    ctx->time_end();
+    ctx->stats.launches++;
+    ctx->stats.keccak_msgs += n_nodes;
+    ctx->stats.keccak_bytes += total;
+    ctx->perms_pending = true;
+    return PHANT_GPU_OK;
+}
+
 // host pointers + deduplicated witness: distinct nodes are hashed once, chains are index lists (one shot, no chunking:
 // a chunk of proofs does not map to a contiguous range of nodes)
 static int verify_dedup_host(phant_gpu_ctx* ctx, const phant_gpu_proof_batch* in, uint64_t* accept_bitmap, uint8_t* status,
@@ -379,6 +423,9 @@ extern "C" int phant_gpu_verify_proofs(phant_gpu_ctx* ctx, const phant_gpu_proof
                 CU(cudaStreamSynchronize(ctx->stream));
             }
         }
+        if (!in->node_index && fused_path(ctx, in->nodes))
+            return verify_fused(ctx, in->nodes, in->node_off, in->proof_first, np, n_nodes, total, in->keys32, in->roots32, in->n_roots,
+                                accept_bitmap, status, val_off, val_len, (const PeerOut*)ctx->walk_peer, true); // asynchronous, as below
         if (int rc = ctx->d_digests.reserve(ctx, 32 * n_nodes + 32)) return rc;
         if (int rc = ctx->d_summary.reserve(ctx, 4 * n_nodes + 32)) return rc;
         if (int rc = ctx->hash_csr(in->nodes, in->node_off, n_nodes, total, (uint8_t*)ctx->d_digests.ptr, (uint32_t*)ctx->d_summary.ptr)) return rc;
@@ -405,8 +452,11 @@ extern "C" int phant_gpu_verify_proofs(phant_gpu_ctx* ctx, const phant_gpu_proof
     if (int rc = ctx->d_first.reserve(ctx, 8 * (np + 1))) return rc;
     if (int rc = ctx->d_keys.reserve(ctx, 32 * np)) return rc;
     if (int rc = ctx->d_roots.reserve(ctx, 32 * in->n_roots)) return rc;
-    if (int rc = ctx->d_digests.reserve(ctx, 32 * n_nodes + 32)) return rc;
-    if (int rc = ctx->d_summary.reserve(ctx, 4 * n_nodes + 32)) return rc;
+    const bool fused = fused_path(ctx, (const uint8_t*)ctx->d_msgs.ptr);
+    if (!fused) { // the two-pass path keeps every digest and summary of the batch
+        if (int rc = ctx->d_digests.reserve(ctx, 32 * n_nodes + 32)) return rc;
+        if (int rc = ctx->d_summary.reserve(ctx, 4 * n_nodes + 32)) return rc;
+    }
     if (int rc = ctx->d_bitmap.reserve(ctx, bm_bytes)) return rc;
     if (int rc = ctx->d_status.reserve(ctx, np)) return rc;
     if (val_off) if (int rc = ctx->d_voff.reserve(ctx, 8 * np)) return rc;
@@ -466,6 +516,19 @@ extern "C" int phant_gpu_verify_proofs(phant_gpu_ctx* ctx, const phant_gpu_proof
         CU(cudaEventRecord(ctx->chunk_events[chunk], cs));
         CU(cudaStreamWaitEvent(s, ctx->chunk_events[chunk], 0));
         nvtxRangePop();
+        if (fused) {
+            if (int rc = verify_fused(ctx, d_nodes, d_noff, d_pfirst + p0, p1 - p0, n1 - n0, b1 - b0, (const uint8_t*)ctx->d_keys.ptr + 32 * p0,
+                                      (const uint8_t*)ctx->d_roots.ptr + (in->n_roots == 1 ? 0 : 32 * p0), in->n_roots,
+                                      (uint64_t*)ctx->d_bitmap.ptr + p0 / 64, (uint8_t*)ctx->d_status.ptr + p0,
+                                      val_off ? (uint64_t*)ctx->d_voff.ptr + p0 : nullptr, val_len ? (uint32_t*)ctx->d_vlen.ptr + p0 : nullptr,
+                                      nullptr, false)) {
+                cudaStreamSynchronize(cs); // as below: no DMA on the caller's buffers after we return
+                cudaStreamSynchronize(s);
+                return rc;
+            }
+            p0 = p1;
+            continue;
+        }
         if (int rc = ctx->hash_csr(d_nodes, d_noff + n0, n1 - n0, b1 - b0, (uint8_t*)ctx->d_digests.ptr + 32 * n0,
                                    (uint32_t*)ctx->d_summary.ptr + n0)) {
             cudaStreamSynchronize(cs); // as above: no DMA on the caller's buffers after we return

@@ -13,11 +13,13 @@ cudaError_t launch_keccak(cudaStream_t s, int device, KeccakVariant variant, con
                           const uint32_t* order, uint64_t n, uint8_t* out, uint32_t* summary /*nullable*/,
                           const uint64_t* len = nullptr /*nullable: message m = msgs[off[m] .. off[m] + len[m])*/);
 // regrouping by permutation count (stable 16-bucket counting sort, two launches): classify fills hist[blocks][16], counts the
-// permutations and leaves global start positions in hist; regroup writes `order`
+// permutations (perms: nullable) and leaves global start positions in hist; regroup writes `order`.  Items are messages
+// (first == nullptr) or proofs of a CSR chain (item i = nodes first[i] .. first[i+1] of `off`).
 uint64_t keccak_regroup_scratch_bytes(int device, uint64_t n);
-cudaError_t launch_keccak_classify(cudaStream_t s, int device, const uint64_t* off, uint64_t n, uint32_t* hist, uint32_t* ticket,
-                                   unsigned long long* perms);
-cudaError_t launch_keccak_regroup(cudaStream_t s, int device, const uint64_t* off, uint64_t n, const uint32_t* start, uint32_t* order);
+cudaError_t launch_keccak_classify(cudaStream_t s, int device, const uint64_t* off, const uint64_t* first /*nullable*/, uint64_t n,
+                                   uint32_t* hist, uint32_t* ticket, unsigned long long* perms /*nullable*/);
+cudaError_t launch_keccak_regroup(cudaStream_t s, int device, const uint64_t* off, const uint64_t* first /*nullable*/, uint64_t n,
+                                  const uint32_t* start, uint32_t* order);
 
 // Peer-memory epilogue of the proof walk (comm.cu "peer transport"): every warp stores its ballot word straight into the
 // gathered bitmap of EVERY rank of the node through NVLink peer mappings (lane r < world stores to rank r: one predicated
@@ -39,6 +41,16 @@ cudaError_t launch_walk(cudaStream_t s, int device, uint64_t n_proofs, const uin
                         const uint64_t* node_index /*nullable*/, const uint64_t* proof_first, const uint8_t* keys32, const uint8_t* roots32, uint64_t n_roots,
                         const uint8_t* digests, const uint32_t* summary /*nullable*/, uint64_t* bitmap, uint8_t* status,
                         uint64_t* val_off, uint32_t* val_len, const PeerOut* peer = nullptr /*nullable: fused gather over peer memory*/);
+
+// verify_fused.cu: hash and walk every proof of a CSR chain in one kernel (one lane per proof, `order`: nullable proof
+// order from the regrouping above); counts its permutations into *perms (one atomic per warp).  The bitmap must be zeroed
+// by the caller (a regrouped warp sets the bits of proofs it does not hold a whole word of with atomicOr); with `peer` the
+// words go to every rank's gathered bitmap and `order` must be nullptr.
+bool verify_fused_supported(const uint8_t* nodes);
+cudaError_t launch_verify_fused(cudaStream_t s, int device, uint64_t n_proofs, const uint8_t* nodes, const uint64_t* node_off,
+                                const uint64_t* proof_first, const uint32_t* order, const uint8_t* keys32, const uint8_t* roots32,
+                                uint64_t n_roots, uint64_t* bitmap, uint8_t* status, uint64_t* val_off, uint32_t* val_len,
+                                unsigned long long* perms, const PeerOut* peer = nullptr);
 
 cudaError_t launch_peer_collect(cudaStream_t s, const unsigned long long* ready, uint32_t world, unsigned long long step, const void* src, void* dst,
                                 uint64_t bytes, const PeerOut& sig);

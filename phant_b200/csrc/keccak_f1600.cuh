@@ -171,19 +171,26 @@ __device__ __forceinline__ uint32_t lds32(uint32_t saddr)
 #else // test harness (tests/hostcheck): "shared memory" is a host array, addresses are offsets into it
 __device__ __forceinline__ uint32_t lds32(uint32_t saddr) { uint32_t v; memcpy(&v, PHANT_HOST_SMEM + saddr, 4); return v; }
 #endif
+// `aligned`: the caller knows sa % 4 == 0 for every lane of the warp (a warp-uniform test), so the words are the block's bytes
+// as they are and the 34 funnel shifts are skipped.  Only the absorb is duplicated; the permutation stays one copy.
 template <int UNROLL, bool DIGEST_ONLY = false>
-__device__ __forceinline__ void absorb_full_smem(uint64_t (&st)[25], uint32_t sa)
+__device__ __forceinline__ void absorb_full_smem(uint64_t (&st)[25], uint32_t sa, bool aligned = false)
 {
-    const uint32_t a4 = sa & ~3u, sh = (sa & 3u) * 8;
-    uint32_t w[2 * KECCAK_RATE_WORDS + 1];
+    if (aligned) {
 #pragma unroll
-    for (int j = 0; j < 2 * KECCAK_RATE_WORDS; ++j) w[j] = lds32(a4 + 4 * j);
-    w[2 * KECCAK_RATE_WORDS] = sh ? lds32(a4 + 4 * 2 * KECCAK_RATE_WORDS) : 0; // holds block bytes only when skewed
+        for (int k = 0; k < KECCAK_RATE_WORDS; ++k) st[k] ^= ((uint64_t)lds32(sa + 8 * k + 4) << 32) | lds32(sa + 8 * k);
+    } else {
+        const uint32_t a4 = sa & ~3u, sh = (sa & 3u) * 8;
+        uint32_t w[2 * KECCAK_RATE_WORDS + 1];
 #pragma unroll
-    for (int k = 0; k < KECCAK_RATE_WORDS; ++k) {
-        const uint32_t lo = __funnelshift_r(w[2 * k], w[2 * k + 1], sh);
-        const uint32_t hi = __funnelshift_r(w[2 * k + 1], w[2 * k + 2], sh);
-        st[k] ^= ((uint64_t)hi << 32) | lo;
+        for (int j = 0; j < 2 * KECCAK_RATE_WORDS; ++j) w[j] = lds32(a4 + 4 * j);
+        w[2 * KECCAK_RATE_WORDS] = sh ? lds32(a4 + 4 * 2 * KECCAK_RATE_WORDS) : 0; // holds block bytes only when skewed
+#pragma unroll
+        for (int k = 0; k < KECCAK_RATE_WORDS; ++k) {
+            const uint32_t lo = __funnelshift_r(w[2 * k], w[2 * k + 1], sh);
+            const uint32_t hi = __funnelshift_r(w[2 * k + 1], w[2 * k + 2], sh);
+            st[k] ^= ((uint64_t)hi << 32) | lo;
+        }
     }
     keccak_f1600<UNROLL, DIGEST_ONLY>(st);
 }
@@ -220,7 +227,7 @@ __device__ __forceinline__ void absorb_final_smem_masked(uint64_t (&st)[25], uin
 }
 // `room` = bytes from `sa` to the end of the lane's slot
 template <int UNROLL>
-__device__ __forceinline__ void absorb_final_smem(uint64_t (&st)[25], uint32_t sa, uint32_t rem, uint32_t room)
+__device__ __forceinline__ void absorb_final_smem(uint64_t (&st)[25], uint32_t sa, uint32_t rem, uint32_t room, bool aligned = false)
 {
     if (room < KECCAK_RATE + 4) { absorb_final_smem_masked<UNROLL>(st, sa, rem); return; }
     const uint32_t a4 = sa & ~3u, s = sa & 3u;
@@ -232,7 +239,7 @@ __device__ __forceinline__ void absorb_final_smem(uint64_t (&st)[25], uint32_t s
     sts32_(a4 + 4 * q0, w0);
     for (uint32_t q = q0 + 1; q < q1; ++q) sts32_(a4 + 4 * q, 0u);
     if (q1 > q0) sts32_(a4 + 4 * q1, 0x80u << (8 * b1));        // bytes above b1 lie past the block and are never used
-    absorb_full_smem<UNROLL, true>(st, sa);                     // last permutation: only the digest lanes are finished
+    absorb_full_smem<UNROLL, true>(st, sa, aligned);            // last permutation: only the digest lanes are finished
 }
 
 // Whole-message Keccak-256 from global or shared memory (generic pointer), any alignment.

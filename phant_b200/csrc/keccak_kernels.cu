@@ -22,6 +22,7 @@
 #include "common.cuh"
 #include "keccak_f1600.cuh"
 #include "node_summary.cuh"
+#include "stage.cuh"
 
 #include <stdlib.h>
 #include <string.h>
@@ -51,54 +52,6 @@ keccak256_direct_kernel(const uint8_t* __restrict__ msgs, const uint64_t* __rest
 // ------------------------------------------------------------------------------------------------
 // staged: bulk-copy engine -> per-lane shared-memory slot -> registers
 // ------------------------------------------------------------------------------------------------
-// window = what one bulk copy brings in: BLOCKS rate blocks + 15 bytes of skew, rounded to 16 x odd so that the 16-byte
-// windows of a quarter warp fall in distinct banks.  The lane's slot is 32 bytes longer than the window (still 16 x odd):
-// the final block is padded IN the slot (absorb_final_smem), which needs 140 bytes behind the block's start; with only
-// the window, a last block that follows BLOCKS-1 full ones at a skew of 13..15 did not fit and took the masked path --
-// 3 of 16 such messages at arbitrary alignment, and because lanes of one warp then split between the two paths the warp
-// paid for both (C3: 3.93 -> 3.30 G perm/s).  + 16 bytes behind the last slot: the reader may touch 4 bytes past a message.
-constexpr int stage_window(int blocks)
-{
-    int s = (blocks * KECCAK_RATE + 15 + 15) / 16;
-    if (s % 2 == 0) ++s;
-    return 16 * s;
-}
-constexpr int stage_slot(int blocks) { return stage_window(blocks) + 32; }
-constexpr int stage_smem(int blocks, int warps) { return 128 + warps * 32 * stage_slot(blocks) + 16; }
-static_assert(stage_smem(4, 12) <= 232448, "default shape must fit the 227 KB a CTA may opt into");
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "LAB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-        "@P1 bra DONE;\n"
-        "bra LAB_WAIT;\n"
-        "DONE:\n"
-        "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 template <int UNROLL, int BLOCKS, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32)
 keccak256_staged_kernel(const uint8_t* __restrict__ msgs, const uint64_t* __restrict__ off,
@@ -148,6 +101,8 @@ keccak256_staged_kernel(const uint8_t* __restrict__ msgs, const uint64_t* __rest
             }
             mbar_wait(bar, parity);
             parity ^= 1;
+            // every lane's node starts at a multiple of 4 bytes (C2: always): absorb without the byte-skew funnel shifts
+            const bool aligned = __all_sync(0xffffffffu, done || (cur & 3) == 0);
             if (!done) {
                 const uint32_t skew = (uint32_t)(cur - a0);
                 const uint64_t in_slot = cs - skew; // message bytes present in the slot (cs == 0 -> need == 0)
@@ -157,11 +112,11 @@ keccak256_staged_kernel(const uint8_t* __restrict__ msgs, const uint64_t* __rest
                 const uint32_t nfull = (uint32_t)(avail / KECCAK_RATE);
                 uint32_t sa = slot_s + skew;
                 for (uint32_t b = 0; b < nfull; ++b) {
-                    absorb_full_smem<UNROLL>(st, sa);
+                    absorb_full_smem<UNROLL>(st, sa, aligned);
                     sa += KECCAK_RATE;
                 }
                 if (avail == need) { // the message ends inside this window: pad and finish
-                    absorb_final_smem<UNROLL>(st, sa, (uint32_t)(avail - (uint64_t)nfull * KECCAK_RATE), slot_s + SLOT - sa);
+                    absorb_final_smem<UNROLL>(st, sa, (uint32_t)(avail - (uint64_t)nfull * KECCAK_RATE), slot_s + SLOT - sa, aligned);
                     done = true;
                 } else {
                     cur += (uint64_t)nfull * KECCAK_RATE;
@@ -260,8 +215,11 @@ keccak256_warp_kernel(const uint8_t* __restrict__ msgs, const uint64_t* __restri
 // ------------------------------------------------------------------------------------------------
 // regrouping by permutation count: a stable 16-bucket counting sort in two launches of our own
 // ------------------------------------------------------------------------------------------------
-// Lanes of a warp run in lockstep, so a warp costs max(permutations) over its 32 messages: `order` lists the message
-// indices class by class (heaviest first; class = 15 - min(15, rate blocks)), each class in ascending index order.
+// Lanes of a warp run in lockstep, so a warp costs max(permutations) over its 32 items: `order` lists the item indices class
+// by class (heaviest first), each class in ascending index order.  An item is either one message (`first` == nullptr: class =
+// 15 - min(15, permutations - 1)) or one proof of a CSR chain, items i = nodes first[i] .. first[i+1] (the fused verify kernel:
+// one lane hashes and walks a whole chain; class = 15 - min(15, (permutations - 1) / 4), one class per full branch node, so
+// that chains of depth 4 .. 12 fall in distinct classes).
 //   launch 1  keccak_class_kernel: block b histograms its contiguous chunk of messages (hist[b][16]) and adds the
 //             chunk's permutation count to the statistics; the LAST block to finish turns the matrix into global start
 //             positions in place (class-major exclusive scan: start[b][c] = sum of classes < c + sum over blocks < b);
@@ -270,15 +228,23 @@ keccak256_warp_kernel(const uint8_t* __restrict__ msgs, const uint64_t* __restri
 // No library sort, no temporary storage beyond 64 bytes per block, deterministic output.
 constexpr int CLS_THREADS = 256, CLS_WARPS = CLS_THREADS / 32;
 
-__device__ __forceinline__ uint32_t keccak_class_of(uint64_t len)
+// permutations of item i (see above)
+__device__ __forceinline__ uint64_t keccak_item_perms(const uint64_t* __restrict__ off, const uint64_t* __restrict__ first, uint64_t i)
 {
-    const uint64_t nb = len / KECCAK_RATE + 1; // permutations of this message
-    return (uint32_t)(15 - (nb > 16 ? 15 : nb - 1));
+    if (!first) return (off[i + 1] - off[i]) / KECCAK_RATE + 1;
+    uint64_t nb = 0;
+    for (uint64_t j = first[i], e = first[i + 1]; j < e; ++j) nb += (off[j + 1] - off[j]) / KECCAK_RATE + 1;
+    return nb;
+}
+__device__ __forceinline__ uint32_t keccak_class_of(uint64_t nb, bool proofs)
+{
+    const uint64_t c = proofs ? (nb ? (nb - 1) / 4 : 0) : nb - 1;
+    return (uint32_t)(15 - (c > 15 ? 15 : c));
 }
 
 __global__ void __launch_bounds__(CLS_THREADS)
-keccak_class_kernel(const uint64_t* __restrict__ off, uint64_t n, uint64_t chunk, uint32_t* __restrict__ hist /* gridDim.x * 16 */,
-                    uint32_t* __restrict__ ticket, unsigned long long* __restrict__ perms)
+keccak_class_kernel(const uint64_t* __restrict__ off, const uint64_t* __restrict__ first, uint64_t n, uint64_t chunk,
+                    uint32_t* __restrict__ hist /* gridDim.x * 16 */, uint32_t* __restrict__ ticket, unsigned long long* __restrict__ perms)
 {
     __shared__ uint32_t h[16];
     __shared__ uint32_t cls_total[16];
@@ -292,15 +258,15 @@ keccak_class_kernel(const uint64_t* __restrict__ off, uint64_t n, uint64_t chunk
         const bool valid = i < hi;
         uint32_t c = 16;
         if (valid) {
-            const uint64_t len = off[i + 1] - off[i];
-            c = keccak_class_of(len);
-            local += len / KECCAK_RATE + 1;
+            const uint64_t nb = keccak_item_perms(off, first, i);
+            c = keccak_class_of(nb, first != nullptr);
+            local += nb;
         }
         const uint32_t peers = __match_any_sync(0xffffffffu, c);
         if (valid && (threadIdx.x & 31) == (uint32_t)(__ffs(peers) - 1)) atomicAdd(&h[c], __popc(peers));
     }
     for (int o = 16; o; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
-    if ((threadIdx.x & 31) == 0 && local) atomicAdd(perms, local); // one atomic per warp
+    if ((threadIdx.x & 31) == 0 && local && perms) atomicAdd(perms, local); // one atomic per warp
     __syncthreads();
     if (threadIdx.x < 16) hist[16 * blockIdx.x + threadIdx.x] = h[threadIdx.x];
     __threadfence();
@@ -337,8 +303,8 @@ keccak_class_kernel(const uint64_t* __restrict__ off, uint64_t n, uint64_t chunk
 }
 
 __global__ void __launch_bounds__(CLS_THREADS)
-keccak_regroup_kernel(const uint64_t* __restrict__ off, uint64_t n, uint64_t chunk, const uint32_t* __restrict__ start /* gridDim.x * 16 */,
-                      uint32_t* __restrict__ order)
+keccak_regroup_kernel(const uint64_t* __restrict__ off, const uint64_t* __restrict__ first, uint64_t n, uint64_t chunk,
+                      const uint32_t* __restrict__ start /* gridDim.x * 16 */, uint32_t* __restrict__ order)
 {
     __shared__ uint32_t base[16];
     __shared__ uint32_t wcnt[CLS_WARPS][16];
@@ -350,7 +316,7 @@ keccak_regroup_kernel(const uint64_t* __restrict__ off, uint64_t n, uint64_t chu
         __syncthreads(); // also orders the previous tile's reads of base[] / wcnt[] before they change
         const uint64_t i = i0 + threadIdx.x;
         const bool valid = i < hi;
-        const uint32_t c = valid ? keccak_class_of(off[i + 1] - off[i]) : 16;
+        const uint32_t c = valid ? keccak_class_of(keccak_item_perms(off, first, i), first != nullptr) : 16;
         const uint32_t peers = __match_any_sync(0xffffffffu, c);
         const uint32_t rank = __popc(peers & ((1u << lane) - 1u));
         if (valid && rank == 0) wcnt[warp][c] = __popc(peers);
@@ -467,21 +433,22 @@ uint64_t keccak_regroup_scratch_bytes(int device, uint64_t n)
     class_geometry(device, n ? n : 1, blocks, chunk);
     return 64 * blocks;
 }
-cudaError_t launch_keccak_classify(cudaStream_t s, int device, const uint64_t* off, uint64_t n, uint32_t* hist, uint32_t* ticket,
-                                   unsigned long long* perms)
+cudaError_t launch_keccak_classify(cudaStream_t s, int device, const uint64_t* off, const uint64_t* first, uint64_t n, uint32_t* hist,
+                                   uint32_t* ticket, unsigned long long* perms)
 {
     if (n == 0) return cudaSuccess;
     uint64_t blocks, chunk;
     class_geometry(device, n, blocks, chunk);
-    keccak_class_kernel<<<(unsigned)blocks, CLS_THREADS, 0, s>>>(off, n, chunk, hist, ticket, perms);
+    keccak_class_kernel<<<(unsigned)blocks, CLS_THREADS, 0, s>>>(off, first, n, chunk, hist, ticket, perms);
     return cudaGetLastError();
 }
-cudaError_t launch_keccak_regroup(cudaStream_t s, int device, const uint64_t* off, uint64_t n, const uint32_t* start, uint32_t* order)
+cudaError_t launch_keccak_regroup(cudaStream_t s, int device, const uint64_t* off, const uint64_t* first, uint64_t n, const uint32_t* start,
+                                  uint32_t* order)
 {
     if (n == 0) return cudaSuccess;
     uint64_t blocks, chunk;
     class_geometry(device, n, blocks, chunk);
-    keccak_regroup_kernel<<<(unsigned)blocks, CLS_THREADS, 0, s>>>(off, n, chunk, start, order);
+    keccak_regroup_kernel<<<(unsigned)blocks, CLS_THREADS, 0, s>>>(off, first, n, chunk, start, order);
     return cudaGetLastError();
 }
 

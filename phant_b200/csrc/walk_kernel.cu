@@ -12,39 +12,14 @@
 
 #include <stdlib.h>
 
-#include "walk_one.cuh"  // Item / rlp_item / Bag / walk_one<BAG>
+#include "peer_sync.cuh"
+#include "walk_one.cuh"  // Item / rlp_item_at / Bag / walk_one<BAG>
 
 namespace phant {
 namespace {
 
 // MINB = CTAs of 128 threads the register allocator must fit per SM (8 -> <= 64 registers, 12 -> <= 40, 16 -> <= 32): the
 // walk is latency-bound (dependent loads per node), so residency is traded against spills; measured, see launch_walk
-// system-scope flag accesses for the peer epilogue
-__device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long long* p)
-{
-    unsigned long long v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_sys(unsigned long long* p, unsigned long long v)
-{
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long global_timer_ns()
-{
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-// spin until flags[r] >= value for every r < world (bounded: a peer that died must not hang this GPU)
-__device__ __forceinline__ void wait_flags(const unsigned long long* flags, uint32_t world, unsigned long long value, uint32_t* err)
-{
-    const unsigned long long t0 = global_timer_ns();
-    for (uint32_t r = 0; r < world; ++r)
-        while (ld_acquire_sys(flags + r) < value)
-            if (global_timer_ns() - t0 > 4000000000ull) { *err = 1; return; }
-}
-
 template <bool BAG, int MINB, bool PEER = false>
 __global__ void __launch_bounds__(128, MINB)
 walk_kernel(const Bag bag, uint64_t n_proofs, const uint8_t* __restrict__ nodes, const uint64_t* __restrict__ node_off,

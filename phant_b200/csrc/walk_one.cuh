@@ -25,33 +25,6 @@ struct Item {
     uint32_t pay_len;
 };
 
-// Strict decode of one RLP item at p (avail bytes).  Returns its total size, 0 if malformed.
-__device__ __forceinline__ uint32_t rlp_item(const uint8_t* p, uint32_t avail, Item& it)
-{
-    if (avail == 0) return 0;
-    const uint32_t b = p[0];
-    if (b < 0x80) { it.is_list = 0; it.pay_off = 0; it.pay_len = 1; return 1; }
-    const uint32_t is_list = b >= 0xc0;
-    const uint32_t base_short = is_list ? 0xc0 : 0x80, base_long = is_list ? 0xf7 : 0xb7;
-    it.is_list = is_list;
-    if (b <= base_long) {
-        const uint32_t len = b - base_short;
-        if (1 + len > avail) return 0;
-        if (!is_list && len == 1 && p[1] < 0x80) return 0; // single byte must encode as itself
-        it.pay_off = 1; it.pay_len = len;
-        return 1 + len;
-    }
-    const uint32_t n = b - base_long;
-    if (n > 4 || 1 + n > avail) return 0;
-    if (p[1] == 0) return 0;
-    uint64_t len = 0;
-    for (uint32_t i = 0; i < n; ++i) len = (len << 8) | p[1 + i];
-    if (len <= 55) return 0;
-    if (1 + n + len > avail) return 0;
-    it.pay_off = 1 + n; it.pay_len = (uint32_t)len;
-    return (uint32_t)(1 + n + len);
-}
-
 // 32 bytes at a 16-byte aligned address (digests, roots) as two 128-bit loads
 __device__ __forceinline__ void load32_aligned(const uint8_t* a, uint32_t (&e)[8])
 {
@@ -122,85 +95,120 @@ __device__ uint32_t bag_find(const Bag& bag, const uint8_t* __restrict__ digests
     }
 }
 
-template <bool BAG>
-__device__ int walk_one(const uint8_t* __restrict__ nodes, const uint64_t* __restrict__ node_off,
-                        const uint64_t* __restrict__ node_index, const Bag bag, uint64_t first,
-                        uint64_t last, const uint8_t* __restrict__ key, const uint8_t* __restrict__ root,
-                        const uint8_t* __restrict__ digests, const uint32_t* __restrict__ summary, uint64_t& voff, uint32_t& vlen)
+// ---- the node bytes a walk step reads: a node of the caller's buffer, or the same node staged in a lane's shared-memory slot.
+// Offsets are local to the node; `at(0)` is its first byte.  `load32(o)` reads the 32 bytes at local offset o (inside the
+// node); `tail_ok(e)` says whether `load32_tail(e)`, the 32 bytes ENDING at local offset e, may be read (they may start before
+// the node: the leaf-path compare masks them off).  `abs(o)` is the offset in the caller's node buffer (the value slice returned).
+struct GlobalBytes {
+    const uint8_t* __restrict__ nodes;
+    uint64_t base; // node_off of this node
+    __device__ __forceinline__ uint32_t at(uint32_t o) const { return nodes[base + o]; }
+    __device__ __forceinline__ void load32(uint32_t o, uint32_t (&e)[8]) const { ::phant::load32(nodes + base + o, e); }
+    __device__ __forceinline__ bool tail_ok(uint32_t e) const { return base + e >= 48; } // the 48-byte window stays in the buffer
+    __device__ __forceinline__ void load32_tail(uint32_t e, uint32_t (&t)[8]) const { ::phant::load32(nodes + (base + e - 32), t); }
+    __device__ __forceinline__ uint64_t abs(uint32_t o) const { return base + o; }
+};
+// `p` = the node's first byte in the slot (a generic pointer into shared memory), `skew` = bytes of the slot in front of it
+// (the slot is 16-byte aligned, the node starts at its 16-byte aligned window + skew).  32 bytes = 9 aligned 32-bit words and
+// one funnel shift per word, all inside the slot: a 32-byte read ending at the node's end reaches at most 4 bytes past it.
+struct SlotBytes {
+    const uint8_t* p;
+    uint32_t skew;
+    uint64_t base;
+    __device__ __forceinline__ uint32_t at(uint32_t o) const { return p[o]; }
+    __device__ __forceinline__ void load32(uint32_t o, uint32_t (&e)[8]) const { load32_at(p + o, e); }
+    __device__ __forceinline__ void load32_tail(uint32_t e, uint32_t (&t)[8]) const { load32_at(p + e - 32, t); }
+    __device__ __forceinline__ static void load32_at(const uint8_t* q, uint32_t (&e)[8])
+    {
+        const uintptr_t a = (uintptr_t)q;
+        const uint32_t* w = reinterpret_cast<const uint32_t*>(a & ~(uintptr_t)3);
+        const uint32_t sh = (uint32_t)(a & 3) * 8;
+        uint32_t u[9];
+#pragma unroll
+        for (int i = 0; i < 9; ++i) u[i] = w[i];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) e[i] = __funnelshift_r(u[i], u[i + 1], sh);
+    }
+    __device__ __forceinline__ bool tail_ok(uint32_t e) const { return skew + e >= 32; } // starts inside the slot
+    __device__ __forceinline__ uint64_t abs(uint32_t o) const { return base + o; }
+};
+
+// Strict decode of one RLP item at local offset `at` of a node (avail bytes).  Returns its total size, 0 if malformed.
+template <class Bytes>
+__device__ __forceinline__ uint32_t rlp_item_at(const Bytes& nb, uint32_t at, uint32_t avail, Item& it)
 {
-    voff = 0; vlen = 0;
-    uint32_t expect[8];
-    load32_aligned(root, expect);
-    // the key lives in registers (two 128-bit loads) instead of one byte load per trie level
-    uint32_t kw[8];
-    load32_aligned(key, kw);
-    auto key_nibble = [&](uint32_t q) -> uint32_t { // nibble q of the key, q < 64
-        const uint32_t wi = q >> 3;
-        const uint32_t a01 = (wi & 1) ? kw[1] : kw[0], a23 = (wi & 1) ? kw[3] : kw[2], a45 = (wi & 1) ? kw[5] : kw[4], a67 = (wi & 1) ? kw[7] : kw[6];
-        const uint32_t lo4 = (wi & 2) ? a23 : a01, hi4 = (wi & 2) ? a67 : a45;
-        const uint32_t w = (wi & 4) ? hi4 : lo4;
-        const uint32_t byte = (w >> (8 * ((q >> 1) & 3))) & 0xffu;
-        return (q & 1) ? (byte & 15u) : (byte >> 4);
-    };
-    if (BAG) { // no chain: first/last only feed the "is this the last node" tests, which always pass
-        first = 0;
-        last = 1;
-        if (eq32_const(EMPTY_ROOT, expect)) return ST_ABSENT;
-    } else if (first == last) return eq32_const(EMPTY_ROOT, expect) ? ST_ABSENT : ST_REJECT;
+    if (avail == 0) return 0;
+    const uint32_t b = nb.at(at);
+    if (b < 0x80) { it.is_list = 0; it.pay_off = 0; it.pay_len = 1; return 1; }
+    const uint32_t is_list = b >= 0xc0;
+    const uint32_t base_short = is_list ? 0xc0 : 0x80, base_long = is_list ? 0xf7 : 0xb7;
+    it.is_list = is_list;
+    if (b <= base_long) {
+        const uint32_t len = b - base_short;
+        if (1 + len > avail) return 0;
+        if (!is_list && len == 1 && nb.at(at + 1) < 0x80) return 0; // single byte must encode as itself
+        it.pay_off = 1; it.pay_len = len;
+        return 1 + len;
+    }
+    const uint32_t n = b - base_long;
+    if (n > 4 || 1 + n > avail) return 0;
+    if (nb.at(at + 1) == 0) return 0;
+    uint64_t len = 0;
+    for (uint32_t i = 0; i < n; ++i) len = (len << 8) | nb.at(at + 1 + i);
+    if (len <= 55) return 0;
+    if (1 + n + len > avail) return 0;
+    it.pay_off = 1 + n; it.pay_len = (uint32_t)len;
+    return (uint32_t)(1 + n + len);
+}
 
-    uint32_t pos = 0; // nibbles of the key consumed
-    uint64_t i = first;
-    const uint8_t* cur = nullptr;
-    uint32_t cur_len = 0;
-    bool embedded = false;
+// nibble q of the key, q < 64
+__device__ __forceinline__ uint32_t key_nibble(const uint32_t (&kw)[8], uint32_t q)
+{
+    const uint32_t wi = q >> 3;
+    const uint32_t a01 = (wi & 1) ? kw[1] : kw[0], a23 = (wi & 1) ? kw[3] : kw[2], a45 = (wi & 1) ? kw[5] : kw[4], a67 = (wi & 1) ? kw[7] : kw[6];
+    const uint32_t lo4 = (wi & 2) ? a23 : a01, hi4 = (wi & 2) ? a67 : a45;
+    const uint32_t w = (wi & 4) ? hi4 : lo4;
+    const uint32_t byte = (w >> (8 * ((q >> 1) & 3))) & 0xffu;
+    return (q & 1) ? (byte & 15u) : (byte >> 4);
+}
 
+// One step of the walk: the node whose digest matched `expect` (rule R1, checked by the caller) is interpreted for the key.
+// `len` = node size, `sm` = its summary (node_summary.cuh; 0 = parse it), `last_node` = it is the chain's last node, `pos` =
+// key nibbles consumed so far.  Returns ST_NEXT with `expect` = the hash reference the next node must match, or a terminal
+// status (with voff / vlen set for ST_PRESENT).  Embedded children (< 32 bytes) are walked in place, inside this step.
+enum { ST_NEXT = 4 };
+template <class Bytes>
+__device__ __forceinline__ int walk_node(const Bytes& nb, uint32_t len, uint32_t sm, bool last_node, const uint32_t (&kw)[8], uint32_t& pos,
+                                         uint32_t (&expect)[8], uint64_t& voff, uint32_t& vlen)
+{
+    // fast path: the node is a simple branch (canonical 17-item list, children empty or 32-byte hashes, empty value) and the
+    // summary holds the child mask: no parse, one 32-byte fetch
+    if ((sm & 3u) == 1u && pos < 64) {
+        const uint32_t nibble = key_nibble(kw, pos);
+        ++pos;
+        const uint32_t mask = sm >> 8;
+        if (!((mask >> nibble) & 1u)) return last_node ? ST_ABSENT : ST_REJECT; // empty slot (R3)
+        const uint32_t before = __popc(mask & ((1u << nibble) - 1u));
+        nb.load32(((sm >> 2) & 7u) + 33u * before + (nibble - before) + 1u, expect);
+        return ST_NEXT;
+    }
+    uint32_t cur = 0, cur_len = len; // the item being interpreted: the node, then embedded children
     for (;;) {
-        if (!embedded) {
-            uint64_t ni;
-            if (BAG) {
-                const uint32_t f = bag_find(bag, digests, expect);
-                if (f == BAG_EMPTY) return ST_MISSING; // the witness does not contain the node this reference names
-                ni = f;
-                i = last - 1; // so that ++i below leaves i == last: every terminal test sees "last node"
-            } else {
-                if (i == last) return ST_REJECT; // R3: a hash reference needs a node
-                ni = node_index ? node_index[i] : i; // deduplicated witness: the chain holds node indices
-            }
-            const uint64_t o = node_off[ni];
-            const uint64_t l = node_off[ni + 1] - o;
-            if (l > 0xffffffffull) return ST_REJECT;
-            cur = nodes + o;
-            cur_len = (uint32_t)l;
-            if (!BAG && !eq32_aligned(digests + 32 * ni, expect)) return ST_REJECT; // R1 (bag: the lookup compared it)
-            // fast path: the hash kernel already proved this node a simple branch (canonical 17-item list, children
-            // empty or 32-byte hashes, empty value) and left the child mask: no parse, one 32-byte fetch
-            const uint32_t sm = summary ? summary[ni] : 0;
-            ++i;
-            if ((sm & 3u) == 1u && pos < 64) {
-                const uint32_t nibble = key_nibble(pos);
-                ++pos;
-                const uint32_t mask = sm >> 8;
-                if (!((mask >> nibble) & 1u)) return i == last ? ST_ABSENT : ST_REJECT; // empty slot (R3)
-                const uint32_t before = __popc(mask & ((1u << nibble) - 1u));
-                load32(cur + ((sm >> 2) & 7u) + 33u * before + (nibble - before) + 1u, expect);
-                continue;
-            }
-        }
         Item top;
-        const uint32_t tot = rlp_item(cur, cur_len, top);
+        const uint32_t tot = rlp_item_at(nb, cur, cur_len, top);
         if (tot == 0 || !top.is_list || tot != cur_len) return ST_REJECT; // R2
-        const uint8_t* pay = cur + top.pay_off;
+        const uint32_t pay = cur + top.pay_off;
         const uint32_t pl = top.pay_len;
 
         // one pass over the items: remember item 0, item 1, the item at the key's nibble and item 16
-        const uint32_t want = pos < 64 ? key_nibble(pos) : 16u;
+        const uint32_t want = pos < 64 ? key_nibble(kw, pos) : 16u;
         Item it0{}, it1{}, itw{}, it16{};
         uint32_t off0 = 0, off1 = 0, offw = 0, off16 = 0;
         uint32_t cnt = 0, o = 0;
         while (o < pl) {
             if (cnt == 17) return ST_REJECT;
             Item it;
-            const uint32_t t = rlp_item(pay + o, pl - o, it);
+            const uint32_t t = rlp_item_at(nb, pay + o, pl - o, it);
             if (t == 0) return ST_REJECT;
             if (cnt == 0) { it0 = it; off0 = o; }
             if (cnt == 1) { it1 = it; off1 = o; }
@@ -215,9 +223,9 @@ __device__ int walk_one(const uint8_t* __restrict__ nodes, const uint64_t* __res
         uint32_t child_off;
         if (cnt == 17) {
             if (pos == 64) { // key exhausted: the branch value decides
-                if (it16.is_list || i != last) return ST_REJECT;
+                if (it16.is_list || !last_node) return ST_REJECT;
                 if (it16.pay_len == 0) return ST_ABSENT;
-                voff = (uint64_t)(pay + off16 + it16.pay_off - nodes);
+                voff = nb.abs(pay + off16 + it16.pay_off);
                 vlen = it16.pay_len;
                 return ST_PRESENT;
             }
@@ -225,48 +233,50 @@ __device__ int walk_one(const uint8_t* __restrict__ nodes, const uint64_t* __res
             ++pos;
         } else {
             if (it0.is_list || it0.pay_len == 0) return ST_REJECT;
-            const uint8_t* hp = pay + off0 + it0.pay_off;
-            const uint32_t flag = hp[0] >> 4;
+            const uint32_t hp = pay + off0 + it0.pay_off;
+            const uint32_t h0 = nb.at(hp);
+            const uint32_t flag = h0 >> 4;
             if (flag > 3) return ST_REJECT;
-            if (!(flag & 1) && (hp[0] & 15)) return ST_REJECT;
+            if (!(flag & 1) && (h0 & 15)) return ST_REJECT;
             const uint32_t plen = 2 * (it0.pay_len - 1) + (flag & 1);
             if (plen > 64) return ST_REJECT;
             bool match = 64 - pos >= plen;
             if ((flag & 2) && pos + plen != 64) match = false; // a leaf only proves presence when its path ends the key: nothing to compare otherwise
-            else if (match && (flag & 2) && plen >= 2 && (uint64_t)(hp + it0.pay_len - nodes) >= 48) {
+            else if (match && (flag & 2) && plen >= 2 && nb.tail_ok(hp + it0.pay_len)) {
                 // leaf whose path ends exactly at the key's end: its last plen/2 bytes must equal the key's last plen/2 bytes (and,
                 // for an odd path, the low nibble of hp[0] the nibble before them) -- one wide load instead of a byte loop
                 uint32_t tail[8];
-                load32(hp + it0.pay_len - 32, tail);
-                const uint32_t nb = plen >> 1; // whole bytes compared: key bytes [32 - nb, 32)
+                nb.load32_tail(hp + it0.pay_len, tail);
+                const uint32_t nbytes = plen >> 1; // whole bytes compared: key bytes [32 - nbytes, 32)
                 uint32_t diff = 0;
 #pragma unroll
                 for (int w = 0; w < 8; ++w) {
-                    const int first = 32 - (int)nb - 4 * w; // first compared byte inside word w (<= 0: whole word, >= 4: none)
+                    const int first = 32 - (int)nbytes - 4 * w; // first compared byte inside word w (<= 0: whole word, >= 4: none)
                     const uint32_t m = first <= 0 ? 0xffffffffu : (first >= 4 ? 0u : 0xffffffffu << (8 * first));
                     diff |= (tail[w] ^ kw[w]) & m;
                 }
-                if ((flag & 1) && (hp[0] & 15u) != key_nibble(pos)) diff = 1;
+                if ((flag & 1) && (h0 & 15u) != key_nibble(kw, pos)) diff = 1;
                 match = diff == 0;
             } else if (match) {
                 // path nibble j: odd flag -> nibble 0 is hp[0]&15, then bytes; even -> bytes from hp[1]
                 for (uint32_t j = 0; j < plen; ++j) {
                     const uint32_t q = j + 2 - (flag & 1); // nibble index inside hp (2 nibbles per byte)
-                    const uint32_t pn = (q & 1) ? (hp[q >> 1] & 15u) : (hp[q >> 1] >> 4);
-                    if (pn != key_nibble(pos + j)) { match = false; break; }
+                    const uint32_t hb = nb.at(hp + (q >> 1));
+                    const uint32_t pn = (q & 1) ? (hb & 15u) : (hb >> 4);
+                    if (pn != key_nibble(kw, pos + j)) { match = false; break; }
                 }
             }
             if (flag & 2) { // leaf
-                if (it1.is_list || i != last) return ST_REJECT;
+                if (it1.is_list || !last_node) return ST_REJECT;
                 if (match && pos + plen == 64) {
-                    voff = (uint64_t)(pay + off1 + it1.pay_off - nodes);
+                    voff = nb.abs(pay + off1 + it1.pay_off);
                     vlen = it1.pay_len;
                     return ST_PRESENT;
                 }
                 return ST_ABSENT;
             }
             if (plen == 0) return ST_REJECT;
-            if (!match) return i == last ? ST_ABSENT : ST_REJECT;
+            if (!match) return last_node ? ST_ABSENT : ST_REJECT;
             pos += plen;
             child = it1; child_off = off1;
         }
@@ -275,16 +285,58 @@ __device__ int walk_one(const uint8_t* __restrict__ nodes, const uint64_t* __res
             if (tot_child >= 32) return ST_REJECT;
             cur = pay + child_off;
             cur_len = tot_child;
-            embedded = true;
             continue;
         }
-        embedded = false;
         if (child.pay_len == 0) {
             if (cnt == 2) return ST_REJECT;
-            return i == last ? ST_ABSENT : ST_REJECT;
+            return last_node ? ST_ABSENT : ST_REJECT;
         }
         if (child.pay_len != 32) return ST_REJECT;
-        load32(pay + child_off + child.pay_off, expect);
+        nb.load32(pay + child_off + child.pay_off, expect);
+        return ST_NEXT;
+    }
+}
+
+// The walk of one key over a chain (or, BAG, over the node set), from the digests the hash kernel left: walk_node per node.
+template <bool BAG>
+__device__ int walk_one(const uint8_t* __restrict__ nodes, const uint64_t* __restrict__ node_off,
+                        const uint64_t* __restrict__ node_index, const Bag bag, uint64_t first,
+                        uint64_t last, const uint8_t* __restrict__ key, const uint8_t* __restrict__ root,
+                        const uint8_t* __restrict__ digests, const uint32_t* __restrict__ summary, uint64_t& voff, uint32_t& vlen)
+{
+    voff = 0; vlen = 0;
+    uint32_t expect[8];
+    load32_aligned(root, expect);
+    // the key lives in registers (two 128-bit loads) instead of one byte load per trie level
+    uint32_t kw[8];
+    load32_aligned(key, kw);
+    if (BAG) { // no chain: first/last only feed the "is this the last node" tests, which always pass
+        first = 0;
+        last = 1;
+        if (eq32_const(EMPTY_ROOT, expect)) return ST_ABSENT;
+    } else if (first == last) return eq32_const(EMPTY_ROOT, expect) ? ST_ABSENT : ST_REJECT;
+
+    uint32_t pos = 0; // nibbles of the key consumed
+    uint64_t i = first;
+    for (;;) {
+        uint64_t ni;
+        if (BAG) {
+            const uint32_t f = bag_find(bag, digests, expect);
+            if (f == BAG_EMPTY) return ST_MISSING; // the witness does not contain the node this reference names
+            ni = f;
+            i = last - 1; // so that ++i below leaves i == last: every terminal test sees "last node"
+        } else {
+            if (i == last) return ST_REJECT; // R3: a hash reference needs a node
+            ni = node_index ? node_index[i] : i; // deduplicated witness: the chain holds node indices
+        }
+        const uint64_t o = node_off[ni];
+        const uint64_t l = node_off[ni + 1] - o;
+        if (l > 0xffffffffull) return ST_REJECT;
+        if (!BAG && !eq32_aligned(digests + 32 * ni, expect)) return ST_REJECT; // R1 (bag: the lookup compared it)
+        const uint32_t sm = summary ? summary[ni] : 0;
+        ++i;
+        const int st = walk_node(GlobalBytes{nodes, o}, (uint32_t)l, sm, i == last, kw, pos, expect, voff, vlen);
+        if (st != ST_NEXT) return st;
     }
 }
 
