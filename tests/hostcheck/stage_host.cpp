@@ -2,7 +2,9 @@
 // absorb_final_smem with its in-slot padding and masked fallback) compiled as HOST code, with "shared memory" a host array.
 // The control flow around the absorb calls restates keccak256_staged_kernel's loop for ONE lane (window copy of <= WINDOW
 // bytes from the 16-byte aligned address below the cursor, byte skew, full blocks, final block with `room`).
-// stdin: "<pad_front> <hex message>" per line ("-" = empty); stdout: digest.  Nothing in the product links this.
+// stdin: "<pad_front> <hex message>" per line ("-" = empty); stdout: digest.  Argument "aligned": absorb with `aligned` set,
+// as the kernel does when every lane's cursor is a multiple of 4 (a line whose pad_front is not is refused, exit code 2).
+// Nothing in the product links this.
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -24,7 +26,8 @@ constexpr int WINDOW = 16 * (((BLOCKS * KECCAK_RATE + 15 + 15) / 16) | 1); // ro
 constexpr int SLOT = WINDOW + 32;
 static_assert(WINDOW == 560 && SLOT == 592, "keep in step with keccak_kernels.cu");
 
-static void lane(const uint8_t* buf /*16-byte aligned, message at buf+front*/, uint64_t front, uint64_t len, uint8_t out[32], int* used_masked)
+static void lane(const uint8_t* buf /*16-byte aligned, message at buf+front*/, uint64_t front, uint64_t len, bool aligned, uint8_t out[32],
+                 int* used_masked)
 {
     const uint32_t slot_s = 64; // the lane's slot inside g_smem (16-byte aligned, like the device slots)
     uint64_t cur = front, end = front + len;
@@ -44,11 +47,11 @@ static void lane(const uint8_t* buf /*16-byte aligned, message at buf+front*/, u
         const uint64_t avail = need < in_slot ? need : in_slot;
         const uint32_t nfull = (uint32_t)(avail / KECCAK_RATE);
         uint32_t sa = slot_s + skew;
-        for (uint32_t b = 0; b < nfull; ++b) { absorb_full_smem<2>(st, sa); sa += KECCAK_RATE; }
+        for (uint32_t b = 0; b < nfull; ++b) { absorb_full_smem<2>(st, sa, aligned); sa += KECCAK_RATE; }
         if (avail == need) {
             const uint32_t room = slot_s + SLOT - sa;
             if (room < KECCAK_RATE + 4) ++*used_masked;
-            absorb_final_smem<2>(st, sa, (uint32_t)(avail - (uint64_t)nfull * KECCAK_RATE), room);
+            absorb_final_smem<2>(st, sa, (uint32_t)(avail - (uint64_t)nfull * KECCAK_RATE), room, aligned);
             done = true;
         } else {
             cur += (uint64_t)nfull * KECCAK_RATE;
@@ -57,8 +60,9 @@ static void lane(const uint8_t* buf /*16-byte aligned, message at buf+front*/, u
     memcpy(out, st, 32);
 }
 
-int main()
+int main(int argc, char** argv)
 {
+    const bool aligned = argc > 1 && strcmp(argv[1], "aligned") == 0;
     static char line[1 << 17];
     int masked = 0;
     while (fgets(line, sizeof line, stdin)) {
@@ -73,8 +77,9 @@ int main()
         size_t n = 0;
         if (strcmp(hex, "-") != 0)
             for (; 2 * n + 1 < hl; ++n) { unsigned v; sscanf(hex + 2 * n, "%2x", &v); base[front + n] = (uint8_t)v; }
+        if (aligned && (front & 3)) { fprintf(stderr, "pad_front %u is not a multiple of 4\n", front); return 2; }
         uint8_t dg[32];
-        lane(base, front, n, dg, &masked);
+        lane(base, front, n, aligned, dg, &masked);
         for (int i = 0; i < 32; ++i) printf("%02x", dg[i]);
         printf("\n");
     }

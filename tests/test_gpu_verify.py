@@ -145,8 +145,9 @@ def test_full_size_c2_property(ctx):
 
 
 def test_host_pipeline_many_chunks_and_bad_csr(ctx, oracle):
-    """host-pointer path crosses PCIe in chunks: 40k proofs (> 3 chunks) must give the same verdicts as the
-    oracle; corrupt CSR arrays must be refused with E_INVALID, not read out of bounds."""
+    """host-pointer path crosses PCIe in chunks: 40k proofs (153 MB, so two chunks at the default 128 MB) must give the same
+    verdicts as the oracle; corrupt CSR arrays must be refused with E_INVALID, not read out of bounds.  Many small chunks:
+    test_gpu_fused_layout.py::test_chunked_host_path."""
     from phant_b200 import gpu
     n = 40_000
     o = oracle.synth_c2(n, depth=8, first=7)

@@ -26,7 +26,8 @@ def test_device_header_permutation_on_host(oracle, tmp_path):
 def test_staged_absorb_path_on_host(oracle, tmp_path):
     """the staged kernel's per-lane absorb path (window copy, byte skew, in-slot padding, masked fallback) as host code
     (tests/hostcheck/stage_host.cpp) for every length 0..700 at every byte skew 0..15, plus long messages: digests equal the
-    oracle's, stale slot bytes (0xEE) and neighbouring message bytes (0xA5) never leak in, and the fallback is exercised"""
+    oracle's, stale slot bytes (0xEE) and neighbouring message bytes (0xA5) never leak in, and the fallback is exercised;
+    then the aligned absorb at the skews that allow it (0, 4, 8, 12)"""
     exe = str(tmp_path / "sh")
     subprocess.run(["g++", "-O1", "-std=c++17", "-Wno-unknown-pragmas", "-o", exe, os.path.join(HERE, "hostcheck", "stage_host.cpp")], check=True)
     rng = np.random.default_rng(6)
@@ -43,3 +44,10 @@ def test_staged_absorb_path_on_host(oracle, tmp_path):
         assert got == want, (sk, len(m))
     fallbacks = int(r.stderr.split()[-1])
     assert 0 < fallbacks < len(cases) // 20  # exercised, and rare (only 544..559 bytes left in the window)
+    # the aligned absorb (no funnel shifts), taken when every lane's message starts at a multiple of 4: skews 0, 4, 8, 12
+    aligned = [(sk, m) for sk, m in cases if sk % 4 == 0]
+    stdin = "".join(f"{sk} {m.hex() if m else '-'}\n" for sk, m in aligned)
+    r = subprocess.run([exe, "aligned"], input=stdin, capture_output=True, text=True, check=True)
+    for (sk, m), got in zip(aligned, r.stdout.split("\n")):
+        assert got == memo[m], ("aligned", sk, len(m))
+    assert len(r.stdout.split()) == len(aligned) and int(r.stderr.split()[-1]) > 0
